@@ -6,7 +6,11 @@ minibatch (BASELINE.json configs[1]: 4096x4096, block_size 32, bf16, N=4096 per 
 density 25 % unless --density is given).  Metric = effective TFLOP/s
 = 3 * 2*nnz_blocks*bs^2*N / t  (the reference's own flop accounting, op.cc:102,182).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned (Y, DX, DW) as float32 DIR/{y,dx,dw}.npy (rank 0), so that
+two builds can be compared output for output: inputs and layout are seeded, identical from run to run.  The files hold
+at most 64 MB in all, so a larger output is cut to a fixed, seeded sample of its minibatch rows (DW: of its blocks).
 
 N>1 is launched by torchrun (one rank per GPU): the minibatch axis is sharded (weak
 scaling: every rank holds N=4096 columns), fprop/bprop need no communication and the
@@ -37,6 +41,7 @@ C = K = 4096
 BS = 32
 N_PER_GPU = 4096
 SEED = 1236
+DUMP_BYTES = 64 * 10 ** 6
 
 
 def make_layout(density, cb=C // BS, kb=K // BS, seed=SEED):
@@ -273,6 +278,20 @@ def check_against_oracle(torch, bsmm, lay, axis, W, X, E, y, dx, dw, n_rows=32, 
             "tolerance": "l2_err <= 1e-2 (bf16)"}
 
 
+def dump_outputs(torch, out_dir, arrays):
+    """Save {name: (tensor, dim)} as float32 out_dir/<name>.npy, DUMP_BYTES in all.  A tensor larger than its even share
+    keeps a fixed, seeded, sorted sample of its slices along `dim` (minibatch rows for Y / DX, blocks for DW)."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 128                  # 128: the .npy header
+    for name, (t, dim) in arrays.items():
+        n = t.shape[dim]
+        keep = min(n, share // (4 * (t.numel() // n)))
+        if keep < n:
+            idx = np.sort(np.random.default_rng(SEED).choice(n, keep, replace=False))
+            t = t.index_select(dim, torch.as_tensor(idx, device=t.device))
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -286,7 +305,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--sm-margin", type=int, default=None, help="SMs left free for NCCL when N>1 (default 8 at 2 GPUs, 12 beyond; BSMM_SM_MARGIN wins)")
     ap.add_argument("--blocking-allreduce", action="store_true", help="round-1 behaviour: all-reduce on the compute stream")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's Y, DX, DW to DIR/{y,dx,dw}.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -449,6 +473,9 @@ def main():
             dw_l = bsmm.updat([Xs[li]], [Es[li]], dw_dtype=dw_dtype)
         check = check_against_oracle(torch, bsmm, lay, args.axis, W, Xs[li], Es[li], y_l, dx_l, dw_l)
         check["device_error"] = _lib.device_error()
+        if args.dump_outputs:   # dW as the caller receives it (all-reduced when N>1)
+            dump_outputs(torch, args.dump_outputs, {"y": (y_l, 0 if args.axis else 1), "dx": (dx_l, 0 if args.axis else 1),
+                                                    "dw": (last[2], 0)})
 
     # ---- per-kernel timing (each kernel alone) for the roofline object: cold (rotating inputs > L2) and warm L2
     pk = peaks()
