@@ -286,7 +286,9 @@ int bst_softmax(int x_dtype, int y_dtype, int bsize,
   p.autoregress_at_key = autoregress_at_key;
   p.x = x; p.y = y; p.scale = scale;
   p.batch = batch; p.heads = heads; p.blocks = blocks; p.ctx_blks_q = ctx_blks_q;
-  // TMA-staged kernel: 16-bit tensors, 32 x 32 / 64 x 64 blocks, every row's blocks fit shared memory (<= 16 of them)
+  // TMA-staged kernel: 16-bit tensors, 32 x 32 / 64 x 64 blocks, every row's blocks fit shared memory (<= 16 of them), and
+  // 16-byte-aligned x and y (bulk copies).  Everything else takes the register kernel, which needs x and y aligned to its
+  // vector accesses (softmax_vec_bytes); a misaligned pointer is refused there rather than faulting in the kernel.
   static const bool no_staged = [] { const char* e = getenv("BSMM_SOFTMAX_STAGED"); return e && atoi(e) == 0; }();
   if (!no_staged && x_dtype != BSMM_F32 && y_dtype != BSMM_F32 && (bsize == 32 || bsize == 64) && max_lut >= 1 && max_lut <= 16 &&
       (((uintptr_t)x | (uintptr_t)y) & 15) == 0 && device_info().ok && device_info().cc_major >= 9) {
@@ -301,6 +303,9 @@ int bst_softmax(int x_dtype, int y_dtype, int bsize,
   BSMM_DISPATCH_DTYPE(x_dtype, TX, {
     BSMM_DISPATCH_DTYPE(y_dtype, TY, {
       BSMM_DISPATCH_BSIZE(bsize, BS, {
+        if (!softmax_aligned<TX, BS>(x) || !softmax_aligned<TY, BS>(y))
+          return fail(BSMM_E_ARG, "bst_softmax: x and y must be aligned to %d / %d bytes", softmax_vec_bytes<TX, BS>(),
+                      softmax_vec_bytes<TY, BS>());
         const long long groups = (long long)ctx_blks_q * SoftmaxMap<BS>::GROUPS;
         dim3 grid((unsigned)((groups + SOFTMAX_WARPS - 1) / SOFTMAX_WARPS), heads, batch);
         bst_softmax_kernel<TX, TY, BS><<<grid, SOFTMAX_WARPS * 32, 0, s>>>(p);
@@ -337,6 +342,9 @@ int bst_softmax_grad(int dtype, int dx_dtype, int bsize,
   BSMM_DISPATCH_DTYPE(dtype, T, {
     BSMM_DISPATCH_DTYPE(dx_dtype, TD, {
       BSMM_DISPATCH_BSIZE(bsize, BS, {
+        if (!softmax_aligned<T, BS>(dy) || !softmax_aligned<T, BS>(y) || !softmax_aligned<TD, BS>(dx))
+          return fail(BSMM_E_ARG, "bst_softmax_grad: dy, y and dx must be aligned to %d / %d bytes", softmax_vec_bytes<T, BS>(),
+                      softmax_vec_bytes<TD, BS>());
         const long long groups = (long long)ctx_blks_q * SoftmaxMap<BS>::GROUPS;
         dim3 grid((unsigned)((groups + SOFTMAX_WARPS - 1) / SOFTMAX_WARPS), heads, batch);
         bst_softmax_grad_kernel<T, TD, BS><<<grid, SOFTMAX_WARPS * 32, 0, s>>>(p);

@@ -112,6 +112,11 @@ template <typename T, int EPL> __device__ __forceinline__ void store_vec(T* p, c
   }
 }
 
+// Widest access load_vec / store_vec make to a T tensor: float2 for fp32, EPL packed 16-bit values otherwise.  Every access
+// sits a multiple of this many bytes past the tensor's start, so the start must be aligned to it.
+template <typename T, int BS> constexpr int softmax_vec_bytes() { return sizeof(T) == 4 ? 8 : SoftmaxMap<BS>::EPL * 2; }
+template <typename T, int BS> inline bool softmax_aligned(const void* p) { return ((uintptr_t)p % softmax_vec_bytes<T, BS>()) == 0; }
+
 template <typename TX, typename TY, int BS>
 __global__ void __launch_bounds__(SOFTMAX_WARPS * 32)
 bst_softmax_kernel(const SoftmaxParams p) {

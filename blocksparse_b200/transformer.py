@@ -120,10 +120,26 @@ class BlocksparseTransformer(TransformerCheckers):
         _lib.check(rc, "bst_xn")
         return c
 
+    def _check_sparse(self, t, what):
+        """The kernels index a (batch, heads, blocks, bs, bs) tensor through the LUTs: any other shape reads past it."""
+        if t.dim() != 5 or tuple(t.shape[1:]) != (self.heads, self.blocks, self.blk_size, self.blk_size):
+            raise ValueError("%s has shape %s; expected (batch, %d, %d, %d, %d)"
+                             % (what, tuple(t.shape), self.heads, self.blocks, self.blk_size, self.blk_size))
+
+    @staticmethod
+    def _aligned(t):
+        """Contiguous and 16-byte aligned, as the softmax kernels' vector and bulk accesses need: a view that starts part
+        way into its storage (x[1:], a slice of a flat buffer) is copied."""
+        t = t.contiguous()
+        return t if t.data_ptr() % 16 == 0 else t.clone()
+
     @_lib.guarded
     def _softmax(self, x, scale, use_mask, autoregress_at_key, dtype):
+        self._check_sparse(x, "softmax input")
+        if not x.is_cuda:
+            raise _lib.BsmmError("BlocksparseTransformer needs CUDA tensors (no CPU path)")
         lib = _lib.load()
-        x = x.contiguous()
+        x = self._aligned(x)
         batch = x.shape[0]
         y = torch.empty(x.shape, dtype=dtype, device=x.device)
         d = self._device_luts(x.device)
@@ -139,9 +155,14 @@ class BlocksparseTransformer(TransformerCheckers):
 
     @_lib.guarded
     def _softmax_grad(self, dy, y, scale):
+        self._check_sparse(y, "softmax output")
+        if dy.shape != y.shape:
+            raise ValueError("softmax gradient has shape %s, softmax output %s" % (tuple(dy.shape), tuple(y.shape)))
+        if not (y.is_cuda and dy.is_cuda):
+            raise _lib.BsmmError("BlocksparseTransformer needs CUDA tensors (no CPU path)")
         lib = _lib.load()
-        dy = dy.to(y.dtype).contiguous()
-        y = y.contiguous()
+        dy = self._aligned(dy.to(y.dtype))
+        y = self._aligned(y)
         dx = torch.empty_like(dy)
         d = self._device_luts(y.device)
         rc = lib.bst_softmax_grad(_lib.dtype_code(y.dtype), _lib.dtype_code(dx.dtype), self.blk_size,

@@ -198,6 +198,8 @@ int bst_xn(int a_dtype, int dtype, int bsize, int transpose_a,
  *   autoregress_at_key >= 0 applies the partial-autoregressive rewrite on the fly
  *         (blocksparse/transformer.py:264-274); nt_lut is then required.
  * Limit: max_lut * bsize <= 32768 (bst_op.cc:383).
+ * x and y (bst_softmax_grad: dy, y and dx) must start at an address aligned to the kernels' vector accesses (4 to 16
+ * bytes; 16 always suffices), else BSMM_E_ARG.
  */
 int bst_softmax(int x_dtype, int y_dtype, int bsize,
                 const int32_t* nn_lut, const int32_t* nt_lut, int lut_heads, int blocks, int max_lut,
